@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — rendered frames/s at 1920x1080 with 3M Gaussians (BASELINE.json metric), plus HBM roofline.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A *step* is one pass of the rasterizer hot path (one ``GaussianRasterizer`` forward in SH mode: projection -> binning ->
 per-tile sort -> blend) over one camera of the synthetic 300-frame trajectory (SURVEY §8d configs 3/4), per rank.  With N ranks
@@ -295,6 +295,8 @@ def main():
     ap.add_argument("--gaussians", type=int, default=3_000_000, help="override only for debugging; the metric is quoted at 3M")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="headline + e2e only (skip the secondary measurements)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the headline loop returned (color, depth, "
+                    "alpha, radii) to DIR/<name>.npy as float32, for comparing two builds output by output")
     args = ap.parse_args()
     # stdout carries exactly ONE line, the JSON result: everything else that writes to file descriptor 1 (NCCL's version
     # banner, library chatter) is sent to stderr for the duration of the run
@@ -468,6 +470,11 @@ def main():
     e1.record()
     barrier()
     clocks2 = sampler.report(t_v0, time.time())
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in zip(("color", "depth", "alpha", "radii"), out_ring[(Wm + K - 1) % 2]):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.float().cpu().numpy())
     ms = reduce_ranks(e0.elapsed_time(e1), "max")
     ovf2 = sum(t.stats()["overflow"] for t in tk2)
     if ovf2 or any(r in clocks2["reasons"] for r in ("hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown")):

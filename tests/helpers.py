@@ -1,11 +1,13 @@
 """Shared helpers for the parity tests and tools: run the same seeded inputs through (a) the product CUDA path
-(autovfx_b200, via the C ABI), (b) the compiled reference (oracle/_ref, GPU) and (c) the CPU oracle."""
+(autovfx_b200, via the C ABI), (b) the compiled reference (oracle/_ref, GPU) and (c) the CPU oracle.  The tests compare with
+(b) through ``reference()``: what the reference computed on the test's inputs is stored under tests/golden/ref_*.npz."""
 from __future__ import annotations
 
+import hashlib
 import math
 import os
 import sys
-from typing import Dict, Optional
+from typing import Callable, Dict, Optional
 
 import numpy as np
 import torch
@@ -111,6 +113,76 @@ def run_ref(a: Dict):
                           shs=a["shs"], colors_precomp=a["colors_precomp"], scales=a["scales"], rotations=a["rotations"],
                           cov3D_precomp=a["cov3D_precomp"], sh_degree=a["sh_degree"], scale_modifier=a["scale_modifier"], bg=a["bg"])
     return fw
+
+
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+# A directory: reference() runs the compiled reference and writes what it returned to <dir>/ref_<group>.npz (see
+# tests/golden/make_golden.py); unset, reference() reads tests/golden/ref_<group>.npz.
+RECORD_DIR = os.environ.get("GSR_RECORD_REFERENCE")
+INLINE_BYTES = 1 << 16  # larger arrays are stored as digests unless named in `full`
+_golden: Dict[str, Dict] = {}
+
+
+def _np(x) -> np.ndarray:
+    return x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else np.asarray(x)
+
+
+def digest(x) -> str:
+    a = _np(x)
+    return "sha256:%s:%s:%s" % (a.dtype.str, "x".join(map(str, a.shape)), hashlib.sha256(a.tobytes()).hexdigest())
+
+
+def reference(group: str, key: str, compute: Callable[[], Dict], full=()) -> Dict:
+    """What the reference computed for one test input, {name: np.ndarray or digest string}: ``compute()`` (which runs the
+    reference) when recording, the stored values otherwise.  Arrays up to INLINE_BYTES and those named in ``full`` are stored
+    whole; a larger one as the SHA-256 of its bytes, dtype and shape, which ``same()`` compares bit for bit."""
+    if group not in _golden:
+        path = os.path.join(GOLDEN_DIR, "ref_%s.npz" % group)
+        _golden[group] = {} if RECORD_DIR else dict(np.load(path))
+    st = _golden[group]
+    if RECORD_DIR:
+        for name, v in compute().items():
+            a = _np(v)
+            st[key + "::" + name] = a if (a.nbytes <= INLINE_BYTES or name in full) else np.array(digest(a))
+        os.makedirs(RECORD_DIR, exist_ok=True)
+        np.savez_compressed(os.path.join(RECORD_DIR, "ref_%s.npz" % group), **st)
+    pre = key + "::"
+    out = {k[len(pre):]: v for k, v in st.items() if k.startswith(pre)}
+    assert out, "no stored reference values for %s/%s" % (group, key)
+    return {k: (str(v) if v.dtype.kind == "U" else v) for k, v in out.items()}
+
+
+def same(x, ref) -> bool:
+    """x equals, bit for bit (dtype and shape included), a value returned by reference()."""
+    if isinstance(ref, str):
+        return digest(x) == ref
+    a = _np(x)
+    return a.dtype == ref.dtype and a.shape == ref.shape and np.array_equal(a, ref)
+
+
+def ref_forward(group: str, key: str, a: Dict, names=("color", "depth", "alpha", "radii", "num_rendered"), state=(), full=()) -> Dict:
+    """reference() of one forward of the compiled reference rasterizer on the call arguments ``a``; ``state`` names entries of
+    its internal buffers (oracle.ref_cuda.state) to keep as well."""
+    def compute():
+        fw = run_ref(a)
+        out = {k: fw[k] for k in names}
+        if state:
+            from oracle import ref_cuda
+            rs = ref_cuda.state(a["means3D"].device)
+            out.update({k: rs[k] for k in state})
+        torch.cuda.synchronize()
+        return out
+    return reference(group, key, compute, full=full)
+
+
+def golden_case(name: str) -> Dict:
+    """tests/golden/<name>.npz (the reference's forward + backward on a named case), with grads_<name>.npz when the gradients
+    are stored apart."""
+    gold = dict(np.load(os.path.join(GOLDEN_DIR, name + ".npz")))
+    gp = os.path.join(GOLDEN_DIR, "grads_" + name + ".npz")
+    if os.path.exists(gp):
+        gold.update(np.load(gp))
+    return gold
 
 
 def run_oracle(a: Dict, stop_after="render"):

@@ -1,6 +1,6 @@
 """GPU parity of the activation / per-frame edit row (SURVEY §8 f-3, f-4): gsr_activate_gaussians through autovfx_b200.edit
 against the torch restatement of the reference's transform_gaussians + merge_two_gaussians + GaussianModel activations run
-with torch's CUDA kernels, and the rendered result of a composed scene against the compiled reference rasterizer."""
+with torch's CUDA kernels, and the rendered result of a composed scene against the reference rasterizer's (tests/golden/)."""
 import numpy as np
 import pytest
 import torch
@@ -66,7 +66,7 @@ def test_resident_scene_compose_and_render():
     frame equals the compiled reference rasterizer on the reference-built tensors."""
     from autovfx_b200 import edit, scene
     from autovfx_b200 import rasterizer as R
-    from tests.helpers import run_ref, settings_from
+    from tests.helpers import ref_forward, same, settings_from
     scene_raw, objA, objB = _to(_raw(20_000, 16, 3)), _to(_raw(3_000, 16, 4)), _to(_raw(1_500, 16, 5))
     for r in (scene_raw, objA, objB):
         r["scaling"] = r["scaling"] - 1.0  # small splats
@@ -98,13 +98,15 @@ def test_resident_scene_compose_and_render():
                  bg=torch.zeros(3, device=DEV))
         color, depth, alpha, radii, _ws, _t, _k = R.forward_raw(a["means3D"], a["shs"], None, a["opacities"], a["scales"], a["rotations"], None,
                                                                settings_from(a), sync=True)
-        fw = run_ref(a)  # same composed tensors through the reference rasterizer: bit-identical images
-        assert torch.equal(color, fw["color"]) and torch.equal(depth, fw["depth"]) and torch.equal(radii, fw["radii"])
+        # same composed tensors through the reference rasterizer: bit-identical images
+        fw = ref_forward("edit", "compose_%d" % frame, a, names=("color", "depth", "radii"))
+        assert same(color, fw["color"]) and same(depth, fw["depth"]) and same(radii, fw["radii"])
         b = dict(a)
         for k in ("means3D", "scales", "rotations", "opacities", "shs"):
             b[k] = ref[k].contiguous()
-        fw2 = run_ref(b)  # reference-built tensors (torch ops): agree up to the few last-bit parameter differences
-        assert float((color - fw2["color"]).abs().mean()) < 1e-6 and maxabs(color, fw2["color"]) < 5e-3
+        # reference-built tensors (torch ops): agree up to the few last-bit parameter differences
+        fw2 = torch.from_numpy(ref_forward("edit", "compose_torch_%d" % frame, b, names=("color",), full=("color",))["color"]).to(DEV)
+        assert float((color - fw2).abs().mean()) < 1e-6 and maxabs(color, fw2) < 5e-3
 
 
 def test_edit_errors():

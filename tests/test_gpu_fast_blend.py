@@ -1,5 +1,5 @@
 """Default blend (alpha = ex2.approx(power*log2e + log2 opacity), guarded decisions + exact repair, gsr_blend.cu) against the
-bit-exact blend (GSR_FLAG_EXACT_IMAGES) and the compiled reference: images within BASELINE's 1e-4 (measured: ~1e-6 of the
+bit-exact blend (GSR_FLAG_EXACT_IMAGES) and the reference's CUDA (tests/golden/): images within BASELINE's 1e-4 (measured: ~1e-6 of the
 value), every integer output identical — radii, per-tile lists and n_contrib (the last blended splat of every pixel, i.e. every
 skip / termination decision of the default mode equals the reference's)."""
 import math
@@ -15,11 +15,6 @@ DEV = "cuda:0"
 CASES = ["config1", "small_sh", "small_deg1_m25", "deg3_m25", "deg2_m25", "small_precomp", "big_splats", "dense_tile", "coplanar"]
 
 
-def _have_ref():
-    from oracle import ref_cuda
-    return ref_cuda.available()
-
-
 @pytest.mark.parametrize("name", CASES)
 @pytest.mark.parametrize("for_backward", [False, True])
 def test_fast_equals_exact_decisions_and_is_close(name, for_backward):
@@ -32,8 +27,7 @@ def test_fast_equals_exact_decisions_and_is_close(name, for_backward):
     assert torch.equal(fast["radii"], exact["radii"])
     if for_backward:
         assert torch.equal(nc_fast, exact["views"]["n_contrib"])
-    if _have_ref():
-        Hh.assert_images_close(f_img, Hh.run_ref(a), tol=1e-4)
+    Hh.assert_images_close(f_img, Hh.golden_case(name), tol=1e-4)  # the reference's images on the same case
 
 
 def test_fast_product_frame_six_channels():
@@ -69,10 +63,9 @@ def test_ill_conditioned_and_degenerate_splats_take_the_exact_drain():
     for k in ("color", "depth", "alpha"):
         assert torch.equal(f_img[k], exact[k]), k
     assert torch.equal(nc, exact["views"]["n_contrib"])
-    if _have_ref():
-        ref = Hh.run_ref(a)
-        for k in ("color", "depth", "alpha"):
-            assert torch.equal(exact[k], ref[k]), k
+    ref = Hh.ref_forward("fast_blend", "ill_conditioned", a, names=("color", "depth", "alpha"))
+    for k in ("color", "depth", "alpha"):
+        assert Hh.same(exact[k], ref[k]), k
 
 
 def test_fast_blend_full_size_three_cameras():

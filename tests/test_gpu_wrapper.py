@@ -1,6 +1,6 @@
 """GPU parity of the render() wrapper row (SURVEY §8 a19 / f1 / f2): the 6-channel forward, the per-Gaussian normals, the
-normal maps and the 8-bit hand-off, through the C ABI, against (a) the compiled reference rasterizer called twice the way
-the reference's render() does and (b) the torch restatement of the wrapper's helper functions run with torch's CUDA kernels."""
+normal maps and the 8-bit hand-off, through the C ABI, against (a) the reference rasterizer called twice the way the
+reference's render() does (its outputs stored under tests/golden/) and (b) the torch restatement of the wrapper's helper functions run with torch's CUDA kernels."""
 import math
 import types
 
@@ -9,7 +9,7 @@ import pytest
 import torch
 
 from tests import wrapper_ref as WR
-from tests.helpers import case_inputs, maxabs, resolve, run_ours, run_ref
+from tests.helpers import case_inputs, maxabs, ref_forward, resolve, run_ours, same
 
 pytestmark = pytest.mark.gpu
 
@@ -47,8 +47,8 @@ def test_forward_multi_is_two_passes(name, tight):
     b["shs"], b["colors_precomp"] = None, extra
     second = run_ours(b, tight=tight)
     assert torch.equal(eimg, second["color"])  # bit for bit what a second pass returns
-    ref2 = run_ref(b)
-    assert torch.equal(eimg, ref2["color"])  # ... and what the reference's second pass returns
+    ref2 = ref_forward("wrapper", "second_pass_" + name, b, names=("color",))
+    assert same(eimg, ref2["color"])  # ... and what the reference's second pass returns
 
 
 def test_forward_multi_empty_and_errors():
@@ -196,10 +196,14 @@ def test_render_matches_reference_structure(name):
         out = renderer.render(cam, pc, pipe, a["bg"], scaling_modifier=case["scale_modifier"])
 
     def rasterize(shs=None, colors_precomp=None):
+        """The reference rasterizer's pass: this repository's exact-image pass, checked bit for bit against the reference's."""
         b = dict(a)
         b["shs"], b["colors_precomp"] = shs, colors_precomp
-        fw = run_ref(b)
-        return fw["color"], fw["depth"], fw["alpha"], fw["radii"]
+        fw = run_ours(b, exact=True)
+        ref = ref_forward("wrapper", "render_%s_%s" % (name, "sh" if shs is not None else "precomp"), b, names=("color", "depth", "alpha", "radii"))
+        for k in ("color", "depth", "alpha", "radii"):
+            assert same(fw[k], ref[k]), k
+        return fw["color"].clone(), fw["depth"].clone(), fw["alpha"].clone(), fw["radii"].clone()
     ref = WR.render_two_pass(rasterize, a["means3D"], a["shs"], a["opacities"], a["scales"], a["rotations"], case["sh_degree"],
                              dict(campos=a["campos"], viewmatrix=a["view"], FoVx=cam.FoVx, FoVy=cam.FoVy), a["bg"])
     assert set(out) == {"render", "depth", "normal", "pseudo_normal", "viewspace_points", "visibility_filter", "radii"}

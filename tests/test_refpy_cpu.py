@@ -39,11 +39,14 @@ def test_plyfile_stand_in_round_trips_the_3dgs_layout(tmp_path):
 
 
 def test_reference_modules_import_against_the_drop_in():
-    if not os.path.isdir(ref_py.GS):
-        import pytest
-        pytest.skip("oracle/_ref_py not staged")
-    ns = ref_py.load("ours")
-    import diff_gaussian_rasterization
-    assert ns.rasterizer is diff_gaussian_rasterization  # zero edits: the reference's import line resolves to the drop-in package
-    assert ns.renderer.GaussianRasterizer is diff_gaussian_rasterization.GaussianRasterizer
-    assert callable(ns.renderer.render) and callable(ns.gaussians_utils.transform_gaussians)
+    # the import lines of the reference's callers (gaussian_renderer/__init__.py, scene/gaussian_model.py) resolve to the drop-in
+    ns = {}
+    exec("from diff_gaussian_rasterization import GaussianRasterizationSettings, GaussianRasterizer\n"
+         "from simple_knn._C import distCUDA2", ns)
+    from autovfx_b200 import knn, rasterizer
+    assert ns["GaussianRasterizer"] is rasterizer.GaussianRasterizer and ns["GaussianRasterizationSettings"] is rasterizer.GaussianRasterizationSettings
+    assert ns["distCUDA2"] is knn.distCUDA2
+    if os.path.isdir(ref_py.GS):  # the staged reference modules, where they are staged
+        mods = ref_py.load("ours")
+        assert mods.renderer.GaussianRasterizer is rasterizer.GaussianRasterizer
+        assert callable(mods.renderer.render) and callable(mods.gaussians_utils.transform_gaussians)
