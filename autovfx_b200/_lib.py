@@ -62,7 +62,7 @@ ABI_VERSION = 4
 EXPORTS = ("gsr_abi_version", "gsr_last_error", "gsr_geom_bytes", "gsr_binning_bytes", "gsr_binning_capacity", "gsr_image_bytes",
            "gsr_forward", "gsr_backward", "gsr_mark_visible", "gsr_dist2_bytes", "gsr_dist2", "gsr_get_views",
            "gsr_profile_begin", "gsr_profile_begin_strided", "gsr_profile_end", "gsr_forward_multi", "gsr_axis_normals", "gsr_normal_maps",
-           "gsr_pack_frame", "gsr_activate_gaussians", "gsr_set_option")
+           "gsr_pack_frame", "gsr_activate_gaussians", "gsr_set_option", "gsr_backward_multi")
 
 
 def _load() -> C.CDLL:
@@ -109,6 +109,9 @@ def _load() -> C.CDLL:
     lib.gsr_backward.restype = C.c_int
     lib.gsr_backward.argtypes = [C.POINTER(gsr_frame), C.POINTER(gsr_workspace), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                  C.c_void_p, C.POINTER(gsr_grads), C.c_void_p]
+    lib.gsr_backward_multi.restype = C.c_int
+    lib.gsr_backward_multi.argtypes = [C.POINTER(gsr_frame), C.POINTER(gsr_workspace), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(gsr_grads), C.c_void_p, C.c_void_p]
     lib.gsr_mark_visible.restype = C.c_int
     lib.gsr_mark_visible.argtypes = [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.gsr_dist2.restype = C.c_int

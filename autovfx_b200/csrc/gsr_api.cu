@@ -20,7 +20,8 @@ int normal_maps_impl(int W, int H, const float* normal_img, const float* depth, 
 int pack_frame_impl(int W, int H, const float* rgb, const float* alpha, const float* depth, const float* normal_hwc, float depth_scale,
                     uint8_t* rgba8, uint8_t* normal8, uint8_t* depth8, cudaStream_t st);
 int backward_impl(const gsr_frame* f, const gsr_workspace* ws, const int32_t* radii, const float* out_alpha, const float* dL_dc,
-                  const float* dL_dd, const float* dL_da, const gsr_grads* g, cudaStream_t st);
+                  const float* dL_dd, const float* dL_da, const float* extra, const float* dL_de, float* dL_dextra, const gsr_grads* g,
+                  cudaStream_t st);
 int compose_impl(int N, int M, const float* xyz, const float* f_dc, const float* f_rest, const float* opacity_raw, const float* scaling_raw,
                  const float* rotation_raw, const gsr_object_xform* xform, float* means3D, float* shs, float* opacities, float* scales,
                  float* rotations, cudaStream_t st);
@@ -92,7 +93,16 @@ int gsr_backward(const gsr_frame* frame, const gsr_workspace* ws, const int32_t*
                  const float* dL_dout_color, const float* dL_dout_depth, const float* dL_dout_alpha, const gsr_grads* grads,
                  void* stream) {
     NvtxRange nvtx_("gsr_backward");
-    return gsr::backward_impl(frame, ws, radii, out_alpha, dL_dout_color, dL_dout_depth, dL_dout_alpha, grads, (cudaStream_t)stream);
+    return gsr::backward_impl(frame, ws, radii, out_alpha, dL_dout_color, dL_dout_depth, dL_dout_alpha, nullptr, nullptr, nullptr, grads,
+                              (cudaStream_t)stream);
+}
+
+int gsr_backward_multi(const gsr_frame* frame, const gsr_workspace* ws, const int32_t* radii, const float* out_alpha,
+                       const float* dL_dout_color, const float* dL_dout_depth, const float* dL_dout_alpha, const float* extra_colors,
+                       const float* dL_dout_extra, const gsr_grads* grads, float* dL_dextra_colors, void* stream) {
+    NvtxRange nvtx_("gsr_backward_multi");
+    return gsr::backward_impl(frame, ws, radii, out_alpha, dL_dout_color, dL_dout_depth, dL_dout_alpha, extra_colors, dL_dout_extra,
+                              dL_dextra_colors, grads, (cudaStream_t)stream);
 }
 
 int gsr_mark_visible(int32_t P, const float* means3D, const float* viewmatrix, const float* projmatrix, uint8_t* present,

@@ -10,8 +10,13 @@ frame is
 
     gsr_axis_normals -> gsr_forward_multi (ONE projection/binning/sort/blend pass, 6 colour channels) -> gsr_normal_maps
 
-When gradients are required the reference structure is kept (two autograd rasterizer calls, the second one re-using the
-first one's geometry is not possible under autograd, torch ops for the normal maps), so training code sees the same graph.
+When gradients are required (training) one frame is ONE autograd rasterizer call, ``rasterize_gaussians_multi``: one
+projection/binning/sort/blend forward for the SH colours and the normal colours, one blend backward for both images
+(gsr_backward_multi) and one per-Gaussian backward on the summed contributions.  The per-Gaussian normals
+(``pc.get_normal(dir_pp_normalized) * 0.5 + 0.5``), the normal-image normalisation and the pseudo-normal stencil stay torch ops
+of the caller's graph, as in the reference, so the gradient reaches rotations and scales through ``get_normal``.  ``render``,
+``depth`` and ``radii`` are bit-identical to the reference's two-pass structure; gradients differ only in summation order.
+``set_fused_training(False)`` restores the two-call graph (for A/B comparisons).
 
 Same argument names, return keys and error behaviour as the reference function.
 """
@@ -28,7 +33,21 @@ from ._lib import lib as _L
 from . import rasterizer as R
 from .rasterizer import GaussianRasterizationSettings, GaussianRasterizer
 
-__all__ = ["render", "axis_normals", "normal_maps", "pack_frame", "fov2focal", "TURBO_LUT_BGR"]
+__all__ = ["render", "axis_normals", "normal_maps", "pack_frame", "fov2focal", "TURBO_LUT_BGR", "set_fused_training",
+           "get_fused_training"]
+
+_FUSED_TRAINING = True
+
+
+def set_fused_training(on: bool) -> None:
+    """Default on: under autograd ``render()`` rasterizes the colour and normal images in one ``rasterize_gaussians_multi`` call
+    (one forward and one backward pass).  Off: two ``GaussianRasterizer`` calls, the reference's graph."""
+    global _FUSED_TRAINING
+    _FUSED_TRAINING = bool(on)
+
+
+def get_fused_training() -> bool:
+    return _FUSED_TRAINING
 
 
 def fov2focal(fov: float, pixels: float) -> float:
@@ -255,19 +274,26 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, scaling_modifier:
         return {"render": frame[0:4], "depth": frame[4], "normal": normal_image, "pseudo_normal": pseudo_normal,
                 "viewspace_points": screenspace_points, "visibility_filter": radii > 0, "radii": radii}
 
-    # ---- gradients required: the reference's graph, op for op, on this package's autograd rasterizer
-    rasterizer = GaussianRasterizer(raster_settings=raster_settings)
+    # ---- gradients required: the reference's graph with its two rasterizer calls merged into one (set_fused_training)
     if dir_pp_normalized is None:
         dir_pp = xyz - viewpoint_camera.camera_center.repeat(pc.get_features.shape[0], 1)
         dir_pp_normalized = dir_pp / dir_pp.norm(dim=1, keepdim=True)
-    rendered_image, depth_image, alpha_image, radii = rasterizer(
-        means3D=means3D, means2D=means2D, shs=shs, colors_precomp=colors_precomp, opacities=opacity, scales=scales, rotations=rotations,
-        cov3D_precomp=cov3D_precomp)
-    rendered_image = torch.cat((rendered_image, alpha_image), dim=0)
-    depth_image = depth_image.squeeze(0)
-    normal_normed = pc.get_normal(dir_pp_normalized=dir_pp_normalized) * 0.5 + 0.5
-    normal_image = rasterizer(means3D=means3D, means2D=means2D, shs=None, colors_precomp=normal_normed, opacities=opacity, scales=scales,
-                              rotations=rotations, cov3D_precomp=cov3D_precomp)[0]
+    if _FUSED_TRAINING:
+        normal_normed = pc.get_normal(dir_pp_normalized=dir_pp_normalized) * 0.5 + 0.5
+        rendered_image, depth_image, alpha_image, normal_image, radii = R.rasterize_gaussians_multi(
+            means3D, means2D, shs, colors_precomp, normal_normed, opacity, scales, rotations, cov3D_precomp, raster_settings)
+        rendered_image = torch.cat((rendered_image, alpha_image), dim=0)
+        depth_image = depth_image.squeeze(0)
+    else:
+        rasterizer = GaussianRasterizer(raster_settings=raster_settings)
+        rendered_image, depth_image, alpha_image, radii = rasterizer(
+            means3D=means3D, means2D=means2D, shs=shs, colors_precomp=colors_precomp, opacities=opacity, scales=scales, rotations=rotations,
+            cov3D_precomp=cov3D_precomp)
+        rendered_image = torch.cat((rendered_image, alpha_image), dim=0)
+        depth_image = depth_image.squeeze(0)
+        normal_normed = pc.get_normal(dir_pp_normalized=dir_pp_normalized) * 0.5 + 0.5
+        normal_image = rasterizer(means3D=means3D, means2D=means2D, shs=None, colors_precomp=normal_normed, opacities=opacity, scales=scales,
+                                  rotations=rotations, cov3D_precomp=cov3D_precomp)[0]
     normal_image = (normal_image - 0.5) * 2.
     normal_image = torch.nn.functional.normalize(normal_image.permute(1, 2, 0), p=2, dim=-1)
     c2w = viewpoint_camera.world_view_transform.inverse()

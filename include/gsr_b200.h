@@ -14,6 +14,7 @@
  * and, for the render() wrapper around the two rasterizer passes ("GR/" = sugar/gaussian_splatting/gaussian_renderer/__init__.py):
  *
  *   gsr_forward_multi replaces  both rasterizer(...) calls of one frame           GR/:134-166 (same geometry, second colour set)
+ *   gsr_backward_multi replaces the two rasterizer backward passes of that frame under autograd
  *   gsr_axis_normals  replaces  pc.get_normal(dir_pp_normalized) * 0.5 + 0.5      GR/:131-132,146-147; scene/gaussian_model.py:120-128
  *   gsr_normal_maps   replaces  normal normalisation + depth pseudo normal        GR/:168-191 (depth_pcd2normal GR/:23-38)
  *   gsr_pack_frame    replaces  the per-frame 8-bit conversions before encoding   scene_representation.py:424-438, sugar/render.py:18-22
@@ -208,6 +209,16 @@ typedef struct gsr_grads {
 int gsr_backward(const gsr_frame* frame, const gsr_workspace* ws, const int32_t* radii, const float* out_alpha,
                  const float* dL_dout_color, const float* dL_dout_depth, const float* dL_dout_alpha,
                  const gsr_grads* grads, void* stream);
+
+/* Backward of a gsr_forward_multi(..., extra_colors, out_extra, GSR_FLAG_FOR_BACKWARD) frame on `ws`, called with the same
+ * extra_colors [P,3].  dL_dout_extra [3,H,W] is the gradient of out_extra; the blend backward folds it into the same single
+ * pass, so every gradient in `grads` is the sum of what two gsr_backward calls would return (one for the colour image, one for
+ * a colors_precomp = extra_colors frame with zero depth and alpha gradients), up to summation order.  dL_dextra_colors [P,3]
+ * receives the gradient of extra_colors and is zero-filled by the library.  extra_colors == dL_dout_extra ==
+ * dL_dextra_colors == NULL is gsr_backward; a partial set returns GSR_ERR_INVALID. */
+int gsr_backward_multi(const gsr_frame* frame, const gsr_workspace* ws, const int32_t* radii, const float* out_alpha,
+                       const float* dL_dout_color, const float* dL_dout_depth, const float* dL_dout_alpha, const float* extra_colors,
+                       const float* dL_dout_extra, const gsr_grads* grads, float* dL_dextra_colors, void* stream);
 
 /* present[i] = (view-space z of means3D[i] > 0.2)  — checkFrustum, rasterizer_impl.cu:54-66. */
 int gsr_mark_visible(int32_t P, const float* means3D, const float* viewmatrix, const float* projmatrix,
